@@ -4,6 +4,7 @@ of the headline metric "MPN Groth16 proofs/sec ...; G1 MSM scalars/sec vs HBM ro
 
   python bench.py --gpus N --steps K --warmup W            our arm  (N>1: launched under torchrun)
   python bench.py --impl reference --gpus N --steps K ...   the CPU arm (rank 0 only)
+  ... --dump-outputs DIR    also write the last timed step's result to DIR/g1_msm_sum.npy (see dump_outputs)
 
 A step = one multi-scalar multiplication sum_i [s_i] P_i over synthetic inputs: per GPU 2^20
 uniform Fr scalars (SplitMix64) and 2^20 bases P_i = [k_i] G.  At N GPUs the job is ONE MSM of
@@ -120,6 +121,16 @@ def rank_inputs_seeds(rank):
     return 2 + 7919 * rank, 1 + 104729 * rank
 
 
+def dump_outputs(out_dir, arrays):
+    """Each named array to out_dir/<name>.npy as float64, so that two builds (or the two arms) can be compared output
+    for output.  The bench's result is the 104-byte affine image of the MSM sum (x | y | inf | pad), written one byte
+    per element: exact in float64, and equal images mean equal points."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_reference(args, rank, world):
     """CPU arm: the reference's algorithm (bellman multiexp restated in C — the reference itself is
     Rust on un-vendored crates and cannot be built here) on the host cores this process may use, on
@@ -140,8 +151,10 @@ def run_reference(args, rank, world):
     per_step = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        cref.msm_g1(bases, scalars, cores)
+        result = cref.msm_g1(bases, scalars, cores)
         per_step.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"g1_msm_sum": result})
     dt = sum(per_step) / max(len(per_step), 1)
     val = total / dt
     srt = sorted(per_step)
@@ -255,6 +268,8 @@ def run_ours(args, rank, local_rank, world):
     e2e_ms, _, result_e2e = timed(step_e2e, args.steps, max(args.warmup, 3))
     e2e_step = e2e_ms / args.steps
     assert (result_e2e == result).all(), "e2e and resident paths disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"g1_msm_sum": result})
 
     mpn_multi = None
     if world > 1 and not args.no_mpn:
@@ -489,7 +504,10 @@ def main():
     ap.add_argument("--workload", default="mpn256", choices=["mpn256", "mpn1024"],
                     help="update batch proved in the mpn_groth16 section: production 256-tx batch (2^24) or BASELINE configs[3] 1024-tx (2^26)")
     ap.add_argument("--mpn-steps", type=int, default=3, help="timed update-batch proofs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the MSM sum of the last timed step to DIR/g1_msm_sum.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
